@@ -368,6 +368,29 @@ def real_stream_b200(eng, repeats=3, copies=4):
     return out
 
 
+DUMP_SAMPLES = (1 << 18, 1 << 16)  # luma / chroma samples kept per picture: at most 32 x 4 x (2^18 + 2 x 2^16) B = 48 MB
+
+
+def dump_outputs(eng, step_pics, out_dir):
+    """--dump-outputs: what the last timed step of `value` left for its caller in the DPB, i.e. every picture of that step that
+    no later picture of the step overwrote, in decode order.  Every plane is sampled at the same seeded positions in each
+    picture and written as float32: y.npy (pictures x 2^18), cb.npy and cr.npy (pictures x 2^16), and poc.npy (float64)."""
+    last = {p.params.dst_slot: i for i, p in enumerate(step_pics)}
+    pics = [step_pics[i] for i in sorted(last.values())]
+    rng = np.random.default_rng(0)
+    idx, rows = None, [[], [], []]
+    for p in pics:
+        planes = eng.read_slot(p.params.dst_slot, p.params)
+        if idx is None:
+            idx = [np.sort(rng.choice(pl.size, min(DUMP_SAMPLES[min(c, 1)], pl.size), replace=False)) for c, pl in enumerate(planes)]
+        for c, pl in enumerate(planes):
+            rows[c].append(pl.ravel()[idx[c]].astype(np.float32))
+    os.makedirs(out_dir, exist_ok=True)
+    for c, plane in enumerate(("y", "cb", "cr")):
+        np.save(os.path.join(out_dir, plane + ".npy"), np.stack(rows[c]))
+    np.save(os.path.join(out_dir, "poc.npy"), np.array([p.params.poc for p in pics], np.float64))
+
+
 def run_config(name, eng, torch, dist, stream, a, rank, local_rank, world, headline):
     """Runs one bench configuration on this rank's engine: `value` (records resident in HBM, pictures pipelined over the engine's
     streams), the per-stage one-stream pass behind `roofline`, and `e2e` (host records in, pictures out).  Returns the
@@ -440,6 +463,9 @@ def run_config(name, eng, torch, dist, stream, a, rank, local_rank, world, headl
     ms_res = timed(step_resident, steps)
     launches = eng.launch_count() - l0
     clk = clocks.stop()
+    if headline and a.dump_outputs and rank == 0:
+        v = (counter["step"] - 1) % STEP_VARIANTS
+        dump_outputs(eng, seq[32 * v:32 * (v + 1)], a.dump_outputs)
     # ---- per-stage kernel times: CUDA events around every stage of every picture on the launching stream.  Stages of
     #      different pictures must not overlap for that, so this pass runs the same steps on ONE stream ----
     eng.enable_timing(True)
@@ -529,7 +555,13 @@ def main():
     ap.add_argument("--height", type=int, default=H)
     ap.add_argument("--bit-depth", type=int, default=BD)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write a fixed sample of the pictures the last timed step decoded to DIR/*.npy")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

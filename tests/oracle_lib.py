@@ -2,6 +2,8 @@
 (oracle/_ref/*.so).  TEST INFRASTRUCTURE: imported by tests/, __graft_entry__.smoke() and the
 cpu_baseline / --impl reference legs of bench.py only."""
 import ctypes as C
+import hashlib
+import json
 import os
 import subprocess
 
@@ -40,6 +42,45 @@ def oracle():
 def ref_path(name):
     p = os.path.join(REF_DIR, name)
     return p if os.path.exists(p) else None
+
+
+REF_DIGESTS = os.path.join(ROOT, "tests", "golden", "ref_digests.json")
+
+
+class RefDigest:
+    """SHA-256 over every array one test case compares with the reference, in the order compared.  check() compares it with
+    the digest stored under the test's id in tests/golden/ref_digests.json, so the comparison needs no reference build.
+    Where oracle/_ref is built the tests also compare each array with the live reference; with REF_DIGESTS_OUT=<json file>
+    set, check() then stores the digest (of arrays that all matched the reference) there instead of comparing
+    (tests/golden/make_ref_digests.py)."""
+
+    def __init__(self, key):
+        self.key, self.h = key, hashlib.sha256()
+
+    def add(self, a):
+        import numpy as np
+        a = np.ascontiguousarray(a, dtype=np.int32)  # the digest of an 8-bit plane does not depend on its container type
+        self.h.update(repr(a.shape).encode())
+        self.h.update(a.tobytes())
+
+    def check(self, live):
+        got = self.h.hexdigest()
+        out = os.environ.get("REF_DIGESTS_OUT")
+        if out:
+            assert live, "recording a reference digest needs the live reference (oracle/_ref)"
+            store = json.load(open(out)) if os.path.exists(out) else {}
+            store[self.key] = got
+            with open(out, "w") as f:
+                json.dump(store, f, indent=0, sort_keys=True)
+            return
+        want = json.load(open(REF_DIGESTS)).get(self.key)
+        assert want is not None, f"no reference digest stored for {self.key}"
+        assert got == want, f"{self.key}: the outputs differ from the reference's"
+
+
+def ref_digest(request):
+    """Body of the `digest` fixture of the modules that compare with the reference: one RefDigest per test case."""
+    return RefDigest(f"{request.node.module.__name__}::{request.node.name}")
 
 
 class Oracle:
