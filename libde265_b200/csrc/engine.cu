@@ -2,7 +2,7 @@
 //
 // Per picture: validate the records, build the work lists (MC units, k_residual classes, intra tasks in topological
 // order) and pack everything into one pinned staging buffer on a small host thread pool, ONE host->device copy, then
-//   k_inter_pred8 -> k_residual -> k_mark_pending + k_intra -> k_deblock<V> -> k_deblock<H> -> k_sao_prep + k_sao
+//   k_inter_pred_tma -> k_residual -> k_mark_pending + k_intra -> k_deblock<V> -> k_deblock<H> -> k_sao8 (or k_sao_prep + k_sao)
 // on one of the engine's streams; pictures are pipelined over the streams with per-slot event ordering.
 // Reference pictures never leave the device (DPB slots are device surfaces).
 // There is no CPU fallback: without a CUDA device b200_engine_create fails with B200_ERR_NO_DEVICE.
@@ -284,8 +284,8 @@ struct HostPool {
   }
 };
 
-// One pipeline context = one CUDA stream with everything a picture in flight needs privately.  Pictures are issued
-// round-robin onto the contexts; cross-context ordering comes from per-slot events (SlotSync): a picture waits for the
+// One pipeline context = one CUDA stream with everything a picture in flight needs privately.  Pictures are placed on the
+// contexts by pick_ctx; cross-context ordering comes from per-slot events (SlotSync): a picture waits for the
 // writers of its reference slots and for every earlier reader / writer of its destination slot.  So pictures that do
 // not depend on each other (the B pictures of one hierarchy level, the next intra period's I picture) overlap, and a
 // latency-bound kernel (the intra DAG) of one picture leaves the SMs to the others.
@@ -311,7 +311,7 @@ struct SlotSync {
 #define PLAN_INTRA_PARTS 8
 struct IntraPart {
   uint32_t i0 = 0, i1 = 0, task_base = 0;
-  std::vector<uint32_t> intra_idx, task_of, task_first, task_cell, diag_cnt, diag_off, fill;  // task_cell: region cell x | y << 12 | cells per side << 24 | plane << 28
+  std::vector<uint32_t> intra_idx, task_of, task_cell, fill;  // task_cell: region cell x | y << 12 | cells per side << 24 | plane << 28
 };
 
 struct AsyncState;
@@ -325,21 +325,18 @@ struct b200_engine {
   // runs on (a set is reused when the kernels of the picture that used it B200_STAGE_SETS pictures ago have finished)
   StagingSet stage_pool[B200_STAGE_SETS];
   unsigned next_stage = 0;
-  int n_ctx = 1, next_ctx = 0;
+  int n_ctx = 1;
   // DPB slots are NAMES (what the records' ref_slot / dst_slot say); the pictures live in a pool of physical surfaces.  A picture
   // that writes slot d while earlier pictures on other streams still read (or write) d's current surface gets another, idle
   // surface and the name moves — like register renaming, WAR / WAW hazards between pictures cost nothing, whatever slot policy
   // the host's DPB has (libde265 reuses the first free image, dpb.cc: the hazard is the common case).  Only true (RAW)
-  // dependencies remain.  B200_RENAME=0 keeps every name on one surface.
+  // dependencies remain.
   Surface slot[B200_MAX_PHYS];
   SlotSync ssync[B200_MAX_PHYS];
   int lmap[B200_MAX_SLOTS];       // name -> physical surface, -1: never written
   int owner[B200_MAX_PHYS];       // physical surface -> name it currently carries, -1: free (may still have readers in flight)
   int last_owner[B200_MAX_PHYS];  // the name it carried last (b200_engine_wait_slot also waits for reads of a renamed-away surface)
-  bool rename = true;
   uint64_t pool_geom = 0;  // format of the last picture issued (run_layout)
-  int intra_width_pct = 0;  // off: warps beyond the DAG's width still pay (they run the dependency-free part of later levels ahead: measured)
-  bool sao_legacy = false;  // B200_SAO_LEGACY=1: k_sao for 8-bit pictures too
   uint64_t n_renamed = 0;
   b200_engine()
   {
@@ -365,26 +362,18 @@ struct b200_engine {
   }
   int num_sms = 148;
   long long slot_depth[B200_MAX_SLOTS] = {}, tail_depth[B200_MAX_CTX] = {}, key_depth = 0;  // pick_ctx: dependency depths
-  // one intra task per plane and region in every picture (default).  B200_INTRA_SPLIT=0: pictures with inter prediction merge the
-  // planes of a region into one task — fewer tasks, but each runs its segments in sequence (three dependent L2 round trips);
-  // measured with tickets in level order and 3 CTAs per SM: 4K B picture k_intra 0.25 ms split vs 0.28 ms merged, bench 3382 vs 3210
-  // frames/s
-  bool intra_split_planes = true;
-  bool sched_rr = false;        // B200_SCHED=rr: plain round-robin placement (A/B measurements)
   int n_ind = 2, next_ind = 0, ind_run = 0;  // streams for pictures that read no reference (intra pictures), used round-robin (B200_IND_STREAMS)
   int intra_i_grid = 64;        // grid cap of k_intra for such pictures: the DAG is at most ~160 tasks wide, 64 CTAs (512 warps) cover it and leave the other SMs to the P/B pictures (0: one CTA per SM; B200_INTRA_I_GRID)
   unsigned int *intra_err = nullptr, *intra_err_host = nullptr;  // k_intra gave up a dependency wait (device word; mapped host copy)
   unsigned long long spin_limit_ns = 2000000000ull;              // B200_INTRA_SPIN_LIMIT_MS
   int intra_ctas = 3, poll_ns = 256;  // k_intra: persistent CTAs per SM, back-off cap of the flag polling (B200_INTRA_CTAS / B200_POLL_NS)
-  int region = 16;  // luma size of an intra region task (16 or 8; B200_REGION overrides)
   // B200_TIMELINE=<file>: a CUDA event before and after every launch; the intervals of all streams (ms since the first launch)
   // are appended to the file at b200_engine_sync / destroy: which kernels of which pictures really overlap (tools/timeline.py)
   struct TlEntry { cudaEvent_t e0, e1; const char* name; int poc, ctx; };
   std::vector<TlEntry> tl;
   const char* tl_path = nullptr;
   cudaEvent_t tl_base = nullptr;
-  bool mc_legacy = false;  // B200_MC_LEGACY=1: the first-generation 8-bit MC kernel (k_inter_pred8) for A/B measurements
-  int mc_ctas = 3;         // k_inter_pred_tma: persistent CTAs per SM (B200_MC_CTAS)
+  int mc_ctas = 3;        // k_inter_pred_tma: persistent CTAs per SM (B200_MC_CTAS)
   bool timing = false;
   std::vector<cudaEvent_t> tev;  // timing ring: TIMING_RING pictures x 7 events
   unsigned tcount = 0;           // pictures recorded since enable / reset
@@ -405,8 +394,7 @@ struct b200_engine {
   uint32_t pu_ref_mask[PLAN_PU_PARTS] = {};
   IntraPart ipart[PLAN_INTRA_PARTS];              // plan_intra_*
   std::vector<uint32_t> cell_level[3], task_level, level_off;  // plan_intra_levels
-  int intra_level_order = 2;  // 2: every picture by DAG level, 1: intra pictures only (B200_INTRA_ORDER=level_i), 0: CTB anti-diagonal order everywhere (=diag)
-  std::vector<uint32_t> ctb_count, tiles, tiles_sorted, list_a, list_b, intra_idx, diag_count, task_of, task_first, task_start, task_order;
+  std::vector<uint32_t> ctb_count, tiles, tiles_sorted, list_a, list_b, intra_idx, task_of, task_first, task_start, task_order;
 };
 
 static int async_flush(b200_engine* en);
@@ -453,7 +441,7 @@ struct PicLayout {
   bool direct = false;                   // B200_PIC_RECORDS_PINNED: raw sections are uploaded from raw_src (the caller's arrays)
   const void* raw_src[14] = {};
   size_t raw_sz[14] = {};
-  int intra_levels = 0, intra_width = 0;  // tickets in DAG-level order: number of levels, tasks in the widest level (0: anti-diagonal order)
+  int intra_levels = 0, intra_width = 0;  // intra DAG: number of levels, tasks in the widest level (B200_HOST_PROF prints them)
   bool run_deblock = false, run_sao = false, has_scaling = false;
   b200_pic_params params{};
   uint32_t n_tu = 0;
@@ -531,21 +519,13 @@ extern "C" int b200_engine_create(b200_engine** out, int device)
     en->pool.start(nt);
   }
   if (const char* e = getenv("B200_INTRA_CTAS")) en->intra_ctas = std::max(1, std::min(4, atoi(e)));
-  if (const char* e = getenv("B200_INTRA_SPLIT")) en->intra_split_planes = atoi(e) != 0;
-  if (const char* e = getenv("B200_SCHED")) en->sched_rr = !strcmp(e, "rr");
   if (const char* e = getenv("B200_IND_STREAMS")) en->n_ind = std::max(1, std::min(4, atoi(e)));
   if (const char* e = getenv("B200_INTRA_I_GRID")) en->intra_i_grid = std::max(0, atoi(e));
-  if (const char* e = getenv("B200_RENAME")) en->rename = atoi(e) != 0;
-  if (const char* e = getenv("B200_INTRA_WIDTH_PCT")) en->intra_width_pct = std::max(0, atoi(e));
-  if (const char* e = getenv("B200_SAO_LEGACY")) en->sao_legacy = atoi(e) != 0;
   if (const char* e = getenv("B200_POLL_NS")) en->poll_ns = std::max(32, std::min(100000, atoi(e)));
   if (const char* e = getenv("B200_INTRA_SPIN_LIMIT_MS")) en->spin_limit_ns = 1000000ull * (unsigned long long)std::max(1, std::min(60000, atoi(e)));
-  if (const char* e = getenv("B200_REGION")) en->region = (atoi(e) == 8) ? 8 : 16;
-  if (const char* e = getenv("B200_INTRA_ORDER")) en->intra_level_order = !strcmp(e, "diag") ? 0 : !strcmp(e, "level_i") ? 1 : 2;
   en->tl_path = getenv("B200_TIMELINE");
   en->host_prof = getenv("B200_HOST_PROF") != nullptr;
   if (const char* e = getenv("B200_HOST_PROF_SKIP")) en->host_skip = std::max(0, atoi(e));
-  if (const char* e = getenv("B200_MC_LEGACY")) en->mc_legacy = atoi(e) != 0;
   if (const char* e = getenv("B200_MC_CTAS")) en->mc_ctas = std::max(1, std::min(8, atoi(e)));
   if (const char* e = getenv("B200_STREAMS")) en->n_ctx = std::max(1, std::min(B200_MAX_CTX, atoi(e)));
   for (int k = 0; k < B200_MAX_CTX; k++) {
@@ -652,7 +632,6 @@ extern "C" int b200_engine_set_streams(b200_engine* en, int n)
   int rc = sync_all(en);
   if (rc) return rc;
   en->n_ctx = n;
-  en->next_ctx = 0;
   en->next_ind = 0;
   return B200_OK;
 }
@@ -766,7 +745,7 @@ static int launch_picture(b200_engine* en, PipeCtx& cx, const PicLayout& L, cons
   const bool run_deblock = L.run_deblock, run_sao = L.run_sao;
   if (en->timing) CU(cudaEventRecord(en->ev[1], st));
   if (n_tiles > 0) {
-    if (sizeof(P) == 1 && !en->mc_legacy) {
+    if (sizeof(P) == 1) {
       // reference windows staged by TMA: the tensor maps of the slots this picture reads travel as a kernel parameter
       MctMaps maps;
       memset(&maps, 0, sizeof(maps));
@@ -782,12 +761,10 @@ static int launch_picture(b200_engine* en, PipeCtx& cx, const PicLayout& L, cons
       const uint32_t* tw = (const uint32_t*)(dbase + off[12]);  // tile words, then the batch table
       TL("mc", (k_inter_pred_tma<<<std::min(L.n_batches, en->num_sms * en->mc_ctas), MCT_CTA_THREADS, sizeof(MctShared), st>>>(
                    dp, maps, (const b200_pu*)(dbase + off[0]), (const b200_weight_entry*)(dbase + off[1]), tw, tw + n_tiles, L.n_batches)));
-    } else if (sizeof(P) == 1)
-      k_inter_pred8<<<std::min((n_tiles + MC8_UNITS_PER_CTA - 1) / MC8_UNITS_PER_CTA, en->num_sms * 5), MC8_WARPS * 32, 0, st>>>(dp, refs, (const b200_pu*)(dbase + off[0]), (const b200_weight_entry*)(dbase + off[1]),
-                                                         (const uint32_t*)(dbase + off[12]), n_tiles);
-    else
+    } else {
       k_inter_pred<P><<<(n_tiles + 3) / 4, 128, 0, st>>>(dp, refs, (const b200_pu*)(dbase + off[0]), (const b200_weight_entry*)(dbase + off[1]),
                                                            (const uint32_t*)(dbase + off[12]), n_tiles);
+    }
     en->launches++;
   }
   if (en->timing) CU(cudaEventRecord(en->ev[2], st));
@@ -797,7 +774,6 @@ static int launch_picture(b200_engine* en, PipeCtx& cx, const PicLayout& L, cons
     ra.coeffs = (const b200_coeff*)(dbase + off[5]);
     ra.scaling = L.has_scaling ? dbase + off[11] : nullptr;
     ra.ticket = (unsigned int*)cx.sync_buf;
-    ra.region = en->region;
     ra.poll_ns = en->poll_ns;
     ra.err = en->intra_err;
     ra.err_host = en->intra_err_host;
@@ -844,11 +820,7 @@ static int launch_picture(b200_engine* en, PipeCtx& cx, const PicLayout& L, cons
       int grid = (L.n_task + RC_WARPS - 1) / RC_WARPS;
       // an intra picture's DAG is latency-bound (one CTA per SM is as fast) and should leave room for the pictures it overlaps with
       const bool background = L.ref_mask == 0 && en->n_ctx > 1;
-      int cap = background ? (en->intra_i_grid ? en->intra_i_grid : en->num_sms) : en->num_sms * en->intra_ctas;
-      // tickets in level order: the widest level bounds how many tasks can ever run at once; more warps than that only spin and
-      // keep other pictures' CTAs off the SMs (B200_INTRA_WIDTH_PCT: warps per task of the widest level, in percent; 0 = off)
-      if (L.intra_width > 0 && en->intra_width_pct > 0)
-        cap = std::min(cap, std::max(4, (int)(((long long)L.intra_width * en->intra_width_pct / 100 + RC_WARPS - 1) / RC_WARPS)));
+      const int cap = background ? (en->intra_i_grid ? en->intra_i_grid : en->num_sms) : en->num_sms * en->intra_ctas;
       if (grid > cap) grid = cap;
       TL("intra", (k_intra<P><<<grid, RC_THREADS, sizeof(IntraSmem<P>), st>>>(dp, ra)));
       en->launches++;
@@ -884,7 +856,7 @@ static int launch_picture(b200_engine* en, PipeCtx& cx, const PicLayout& L, cons
   if (run_sao) {
     uint16_t* avail = (uint16_t*)(cx.sync_buf + sync_sao_offset(L.params));
     fa.sao_avail = avail;
-    const bool sao8 = sizeof(P) == 1 && dp.log2ctb >= 5 && !en->sao_legacy;
+    const bool sao8 = sizeof(P) == 1 && dp.log2ctb >= 5;
     if (!sao8) {  // k_sao8 derives the neighbour masks itself
       TL("sao_prep", (k_sao_prep<<<(2 * dp.wctb * dp.hctb + 127) / 128, 128, 0, st>>>(dp, fa, avail)));
       en->launches++;
@@ -973,7 +945,6 @@ static int plan_pus_part(b200_engine* en, const b200_picture* pic, int part, uin
   uint32_t ref_mask = 0;
   size_t count[8] = {0, 0, 0, 0, 0, 0, 0, 0};
   const bool wide = p.bit_depth_luma > 8;  // same rule as the launch_picture<P> dispatch
-  const bool legacy = en->mc_legacy;
   const unsigned pw = p.width, ph = p.height;
   const uint32_t n_weights = pic->n_weights;
   const b200_pu* pus = pic->pus;
@@ -991,13 +962,6 @@ static int plan_pus_part(b200_engine* en, const b200_picture* pic, int part, uin
     if (wide) {  // 16-bit path: <= 16x16 tiles, one warp each (kernels_mc.cuh)
       for (unsigned ty = 0; ty * MC_TILE < h; ty++)
         for (unsigned tx = 0; tx * MC_TILE < w; tx++) *out++ = i | (tx << 20) | (ty << 22);
-    } else if (legacy) {  // first-generation 8-bit path: <= 8x16 units, one quarter-warp each (kernels_mc8.cuh)
-      tiles.resize((size_t)(out - tiles.data()));  // (rare debug path: up to 32 units per PU, keep the simple form)
-      for (unsigned uy = 0; uy * MC8_UH < h; uy++)
-        for (unsigned ux = 0; ux * MC8_UW < w; ux++) tiles.push_back(MC8_UNIT(i, ux, uy));
-      const size_t used = tiles.size();
-      tiles.resize(used + (size_t)(i1 - i - 1) * 32 + 32);
-      out = tiles.data() + used;
     } else {     // 8-bit path: <= 16x16 tiles with their class (kernels_mct.cuh), sorted into class-pure batches by the merge
       const unsigned bi = (l0 && l1) ? MCT_CLASS_BI : 0;
       for (unsigned ty = 0; ty * 16 < h; ty++) {
@@ -1025,7 +989,7 @@ static int plan_pus_merge(b200_engine* en, const b200_picture* pic, PicLayout* L
   L->n_batches = 0;
   for (int part = 0; part < PLAN_PU_PARTS; part++) L->ref_mask |= en->pu_ref_mask[part];
   size_t n_words;
-  if (wide || en->mc_legacy) {
+  if (wide) {
     tiles.clear();
     for (int part = 0; part < PLAN_PU_PARTS; part++) tiles.insert(tiles.end(), en->pu_tiles[part].begin(), en->pu_tiles[part].end());
     n_words = tiles.size();
@@ -1092,18 +1056,13 @@ static inline int tu_check(const TuDims& d, const b200_picture* pic, uint32_t i,
 }
 
 // TU validation, the k_residual classes of the non-intra TUs and the intra work list, in one pass over the TU records.  Intra tasks: the TUs of one plane inside one aligned 16x16-luma / 8x8-chroma region (contiguous per plane in
-// decode order); a TU at least as large as the region is a task of its own.  Tasks are emitted in a topological order: CTB
-// anti-diagonal x + 2y, ties in decode order.  The TU list is cut at CTB boundaries into PLAN_INTRA_PARTS ranges (a region
-// never crosses a CTB, so no task spans two ranges) and the phases A, C, E run per range on the pool threads:
-//   A  per range: intra TUs, their (range-local) task ids, tasks per diagonal          B  serial: task / rank offsets of the ranges
-//   C  per range: rank of every task, TUs per task                                      D  serial: prefix sum -> task_start
+// decode order); a TU at least as large as the region is a task of its own.  Tasks are ranked in a topological order: DAG level,
+// ties in decode order (plan_intra_levels).  The TU list is cut at CTB boundaries into PLAN_INTRA_PARTS ranges (a region never
+// crosses a CTB, so no task spans two ranges) and the phases A, C, E run per range on the pool threads:
+//   A  per range: intra TUs, their (range-local) task ids                               B  serial: task offsets of the ranges, rank of every task
+//   C  per range: TUs per task                                                          D  serial: prefix sum -> task_start
 //   E  per range: list_b (TU indices grouped by task in rank order)
 
-static inline size_t plan_diag_of(const b200_pic_params& p, const b200_tu& tu)
-{
-  const int sh = tu.cidx ? 1 : 0;
-  return (size_t)((tu.x << sh) >> p.log2_ctb_size) + 2 * (size_t)((tu.y << sh) >> p.log2_ctb_size);
-}
 static inline uint32_t plan_ctb_of(const b200_pic_params& p, const b200_tu& tu)
 {
   const int sh = (tu.cidx && tu.cidx <= 2) ? 1 : 0;
@@ -1125,7 +1084,9 @@ static void plan_intra_ranges(b200_engine* en, const b200_picture* pic)
   }
 }
 
-static int plan_intra_A(b200_engine* en, const b200_picture* pic, int k, int n_diag, int wctb, int hctb)
+// One task per plane and region in every picture: merging the planes of a region into one task (fewer tasks, but three dependent
+// L2 round trips each) was measured slower, also in pictures with inter prediction (DESIGN.md §4).
+static int plan_intra_A(b200_engine* en, const b200_picture* pic, int k)
 {
   const b200_pic_params& p = pic->params;
   IntraPart& ip = en->ipart[k];
@@ -1135,49 +1096,10 @@ static int plan_intra_A(b200_engine* en, const b200_picture* pic, int k, int n_d
   la4.clear();
   ip.intra_idx.clear();
   ip.task_of.clear();
-  ip.task_first.clear();
   ip.task_cell.clear();
-  ip.diag_cnt.assign((size_t)n_diag, 0);
-  // Pictures with inter prediction have few, scattered intra blocks: the per-task overhead of k_intra dominates there, so the
-  // small TUs of ALL planes of a region form one task (luma, then Cb, then Cr) when they are at most 16; intra pictures keep
-  // one task per plane (three shorter dependency chains side by side).
-  const bool merged = pic->n_pu > 0 && !en->intra_split_planes;
-  const int lg_region = en->region == 16 ? 4 : 3;
   const TuDims dims = tu_dims(p);
   long long cur_key[3] = {-1, -1, -1};
   uint32_t cur_task[3] = {0, 0, 0};
-  uint32_t run[48];  // merged mode: the small intra TUs of the current region (at most 16 + 4 + 4, sized generously)
-  int n_run = 0;
-  long long run_key = -1;
-  auto new_task = [&](uint32_t first_tu) {
-    const b200_tu& ft = pic->tus[first_tu];
-    ip.task_first.push_back(first_tu);
-    ip.diag_cnt[plan_diag_of(p, ft)]++;
-    const uint32_t sh = ft.cidx ? 1 : 0;  // what plan_intra_levels needs of the task, kept here so that pass reads no TU record
-    const uint32_t R = std::max(1u, ((1u << ft.log2_size) << sh) >> lg_region);
-    ip.task_cell.push_back((((uint32_t)ft.x << sh) >> lg_region) | ((((uint32_t)ft.y << sh) >> lg_region) << 12) | (R << 24) | ((uint32_t)ft.cidx << 28));
-    return (uint32_t)ip.task_first.size() - 1;
-  };
-  auto flush_run = [&]() {
-    if (!n_run) return;
-    int cnt[3] = {0, 0, 0};
-    for (int j = 0; j < n_run; j++) cnt[pic->tus[run[j]].cidx]++;
-    const bool one = n_run <= 16;
-    uint32_t t = 0;
-    if (one) t = new_task(run[0]);
-    for (int c = 0; c < 3; c++) {  // plane by plane, decode order inside a plane
-      if (!cnt[c]) continue;
-      bool first = true;
-      for (int j = 0; j < n_run; j++) {
-        if (pic->tus[run[j]].cidx != c) continue;
-        if (!one && first) t = new_task(run[j]);
-        first = false;
-        ip.intra_idx.push_back(run[j]);
-        ip.task_of.push_back(t);
-      }
-    }
-    n_run = 0;
-  };
   for (uint32_t i = ip.i0; i < ip.i1; i++) {
     const b200_tu& tu = pic->tus[i];
     if (const int rc = tu_check(dims, pic, i, tu)) return rc;
@@ -1189,51 +1111,29 @@ static int plan_intra_A(b200_engine* en, const b200_picture* pic, int k, int n_d
       }
       continue;
     }
-    const int c = tu.cidx, G = en->region >> (c ? 1 : 0), nT = 1 << tu.log2_size;
-    if (merged) {
-      if (nT >= G) {  // a TU at least as large as the region is a task of its own
-        flush_run();
-        run_key = -1;
-        ip.intra_idx.push_back(i);
-        ip.task_of.push_back(new_task(i));
-        continue;
-      }
-      const int sh = c ? 1 : 0;
-      const long long key = (((long long)((tu.y << sh) >> lg_region)) << 20) | ((tu.x << sh) >> lg_region);
-      if (key != run_key || n_run == 48) {
-        flush_run();
-        run_key = key;
-      }
-      run[n_run++] = i;
-      continue;
-    }
+    const int c = tu.cidx, sh = c ? 1 : 0, G = RC_REGION >> sh, nT = 1 << tu.log2_size;
     ip.intra_idx.push_back(i);
-    const long long key = (nT >= G) ? -2 - (long long)i : (((long long)(tu.y >> (lg_region - (c ? 1 : 0)))) << 20) | (tu.x >> (lg_region - (c ? 1 : 0)));
+    const long long key = (nT >= G) ? -2 - (long long)i : (((long long)(tu.y >> (RC_LG_REGION - sh))) << 20) | (tu.x >> (RC_LG_REGION - sh));
     if (key != cur_key[c]) {
       cur_key[c] = key;
-      cur_task[c] = new_task(i);
+      // what plan_intra_levels needs of the task, kept here so that pass reads no TU record
+      const uint32_t R = std::max(1u, ((1u << tu.log2_size) << sh) >> RC_LG_REGION);
+      ip.task_cell.push_back((((uint32_t)tu.x << sh) >> RC_LG_REGION) | ((((uint32_t)tu.y << sh) >> RC_LG_REGION) << 12) | (R << 24) | ((uint32_t)c << 28));
+      cur_task[c] = (uint32_t)ip.task_cell.size() - 1;
     }
     ip.task_of.push_back(cur_task[c]);
   }
-  flush_run();
   return B200_OK;
 }
 
-static void plan_intra_B(b200_engine* en, int n_diag, uint32_t* n_task, uint32_t* n_intra)
+static void plan_intra_B(b200_engine* en, uint32_t* n_task, uint32_t* n_intra)
 {
   uint32_t nt = 0, ni = 0;
   for (int k = 0; k < PLAN_INTRA_PARTS; k++) {
     en->ipart[k].task_base = nt;
-    nt += (uint32_t)en->ipart[k].task_first.size();
+    nt += (uint32_t)en->ipart[k].task_cell.size();
     ni += (uint32_t)en->ipart[k].intra_idx.size();
-    en->ipart[k].diag_off.assign((size_t)n_diag, 0);
   }
-  uint32_t run = 0;
-  for (int d = 0; d < n_diag; d++)
-    for (int k = 0; k < PLAN_INTRA_PARTS; k++) {  // ranges are in decode order: within a diagonal, earlier ranges rank first
-      en->ipart[k].diag_off[d] = run;
-      run += en->ipart[k].diag_cnt[d];
-    }
   *n_task = nt;
   *n_intra = ni;
   en->task_order.resize(nt);
@@ -1241,35 +1141,31 @@ static void plan_intra_B(b200_engine* en, int n_diag, uint32_t* n_task, uint32_t
   en->list_b.resize(ni);
 }
 
-// Ticket order by DAG LEVEL (default; B200_INTRA_ORDER=diag keeps the CTB anti-diagonal order).  A level is assigned per task in
-// ONE pass over the tasks in decode order through a map "region cell (16x16 luma) -> highest level of a task covering it":
+// Ticket order by DAG LEVEL.  A level is assigned per task in ONE pass over the tasks in decode order through a map per plane
+// "region cell (16x16 luma) -> highest level of a task covering it":
 //   level(task) = 1 + max over the cells its TUs may read (the column left of it from one cell above to 2x its height below —
 //   corner, left and bottom-left neighbours — and the row above it to 2x its width — top and top-right), cells not written yet
 //   (decoded later, or not intra) count 0.
 // That is a superset of the true dependencies (availability bits), which is all a valid layering needs: every neighbour a task
 // waits for has a lower level.  Tasks of one level are independent, so with tickets sorted by level the lowest unfinished
 // tickets are exactly the ready tasks: the persistent warps of k_intra hold ready work instead of spinning on tasks far down
-// the anti-diagonal, and the grid is sized to the DAG's width (the widest level) instead of the whole GPU — the other SMs stay
-// free for the pictures it overlaps with.  (The anti-diagonal order is topological too, but of the ~500 consecutive tickets
-// the warps hold only the first task of every CTB chain is ready.)  Intra pictures keep one map per plane (their tasks are
-// per plane); pictures with inter prediction one map (tasks span the planes).
+// the picture.  (A CTB anti-diagonal order is topological too, but of the ~500 consecutive tickets the warps hold only the
+// first task of every CTB chain is ready.)
 static void plan_intra_levels(b200_engine* en, const b200_picture* pic, PicLayout* L, uint32_t n_task)
 {
   const b200_pic_params& p = pic->params;
-  const int lg = en->region == 16 ? 4 : 3;
-  const int cw = (p.width + (1 << lg) - 1) >> lg, ch = (p.height + (1 << lg) - 1) >> lg;
-  const bool per_plane = pic->n_pu == 0 || en->intra_split_planes;
-  for (int c = 0; c < (per_plane ? 3 : 1); c++) en->cell_level[c].assign((size_t)cw * ch, 0);
+  const int cw = (p.width + RC_REGION - 1) >> RC_LG_REGION, ch = (p.height + RC_REGION - 1) >> RC_LG_REGION;
+  for (int c = 0; c < 3; c++) en->cell_level[c].assign((size_t)cw * ch, 0);
   std::vector<uint32_t>& level = en->task_level;
   level.resize(n_task);
   uint32_t max_level = 0;
   for (int k = 0; k < PLAN_INTRA_PARTS; k++) {
     const IntraPart& ip = en->ipart[k];
-    for (size_t t = 0; t < ip.task_first.size(); t++) {
+    for (size_t t = 0; t < ip.task_cell.size(); t++) {
       const uint32_t tc = ip.task_cell[t];
       const int cx = (int)(tc & 0xfff), cy = (int)((tc >> 12) & 0xfff);
       const int R = (int)((tc >> 24) & 0xf);  // cells per side: 1 (region task) or the large TU's size
-      uint32_t* map = en->cell_level[per_plane ? (tc >> 28) : 0].data();
+      uint32_t* map = en->cell_level[tc >> 28].data();
       uint32_t lvl = 0;
       if (cx > 0)
         for (int y = std::max(cy - 1, 0); y < std::min(cy + 2 * R, ch); y++) lvl = std::max(lvl, map[(size_t)y * cw + cx - 1]);
@@ -1281,11 +1177,11 @@ static void plan_intra_levels(b200_engine* en, const b200_picture* pic, PicLayou
       for (int y = cy; y < std::min(cy + R, ch); y++)
         for (int x = cx; x < std::min(cx + R, cw); x++) {
           uint32_t& m = map[(size_t)y * cw + x];
-          if (lvl > m) m = lvl;  // several tasks may cover a cell (planes of a merged region that were split, large chroma TUs)
+          if (lvl > m) m = lvl;  // several tasks may cover a cell (large chroma TUs)
         }
     }
   }
-  // rank = position in (level, decode order): counting sort over the levels; the widest level sizes the grid
+  // rank = position in (level, decode order): counting sort over the levels
   std::vector<uint32_t>& off = en->level_off;
   off.assign((size_t)max_level + 2, 0);
   for (uint32_t t = 0; t < n_task; t++) off[level[t] + 1]++;
@@ -1300,13 +1196,10 @@ static void plan_intra_levels(b200_engine* en, const b200_picture* pic, PicLayou
   L->intra_width = (int)width;
 }
 
-static void plan_intra_C(b200_engine* en, const b200_picture* pic, int k, bool by_level)
+static void plan_intra_C(b200_engine* en, int k)
 {
-  const b200_pic_params& p = pic->params;
-  IntraPart& ip = en->ipart[k];
-  uint32_t* order = en->task_order.data() + ip.task_base;
-  if (!by_level)
-    for (size_t t = 0; t < ip.task_first.size(); t++) order[t] = ip.diag_off[plan_diag_of(p, pic->tus[ip.task_first[t]])]++;
+  const IntraPart& ip = en->ipart[k];
+  const uint32_t* order = en->task_order.data() + ip.task_base;
   uint32_t* ts = en->task_start.data();
   for (size_t j = 0; j < ip.task_of.size(); j++) ts[order[ip.task_of[j]] + 1]++;  // a task belongs to exactly one range: no two threads touch one entry
 }
@@ -1316,8 +1209,8 @@ static void plan_intra_E(b200_engine* en, int k)
   IntraPart& ip = en->ipart[k];
   const uint32_t* order = en->task_order.data() + ip.task_base;
   const uint32_t* ts = en->task_start.data();
-  ip.fill.resize(ip.task_first.size());
-  for (size_t t = 0; t < ip.task_first.size(); t++) ip.fill[t] = ts[order[t]];
+  ip.fill.resize(ip.task_cell.size());
+  for (size_t t = 0; t < ip.task_cell.size(); t++) ip.fill[t] = ts[order[t]];
   uint32_t* lb = en->list_b.data();
   for (size_t j = 0; j < ip.intra_idx.size(); j++) lb[ip.fill[ip.task_of[j]]++] = ip.intra_idx[j];
 }
@@ -1332,14 +1225,13 @@ static void plan_parallel(b200_engine* en, int n, F f)
 
 // The serial glue of the intra planner after phase A has run for every range (also used by plan_and_pack, where phase A runs
 // next to the other planning work).
-static void plan_intra_finish(b200_engine* en, const b200_picture* pic, PicLayout* L, int n_diag)
+static void plan_intra_finish(b200_engine* en, const b200_picture* pic, PicLayout* L)
 {
   uint32_t n_task = 0, n_intra = 0;
-  plan_intra_B(en, n_diag, &n_task, &n_intra);
-  const bool by_level = n_task && (en->intra_level_order == 2 || (en->intra_level_order == 1 && pic->n_pu == 0));
+  plan_intra_B(en, &n_task, &n_intra);
   L->intra_levels = L->intra_width = 0;
-  if (by_level) plan_intra_levels(en, pic, L, n_task);
-  plan_parallel(en, PLAN_INTRA_PARTS, [=](int k) { plan_intra_C(en, pic, k, by_level); });
+  if (n_task) plan_intra_levels(en, pic, L, n_task);
+  plan_parallel(en, PLAN_INTRA_PARTS, [=](int k) { plan_intra_C(en, k); });
   uint32_t* ts = en->task_start.data();
   for (uint32_t t = 0; t < n_task; t++) ts[t + 1] += ts[t];
   plan_parallel(en, PLAN_INTRA_PARTS, [=](int k) { plan_intra_E(en, k); });
@@ -1441,15 +1333,13 @@ static int plan_and_pack(b200_engine* en, const b200_picture* pic, PicLayout* L,
   if (rc) return rc;
   const double t1 = now();
   uint8_t* hb = ss.host;
-  const b200_pic_params& pp = pic->params;
-  const int S = 1 << pp.log2_ctb_size, wctb = (pp.width + S - 1) / S, hctb = (pp.height + S - 1) / S, n_diag = wctb + 2 * hctb;
   en->use_helper = en->helper && pic->n_tu > 200000;  // shadow engines: see b200_engine::helper
   int rc_pu[PLAN_PU_PARTS] = {}, rc_tv[PLAN_TU_PARTS] = {};
   std::string err_pu[PLAN_PU_PARTS], err_tv[PLAN_TU_PARTS];
   plan_intra_ranges(en, pic);
   for (int k = 0; k < PLAN_INTRA_PARTS; k++)  // the longest items first: TU validation + residual classes + intra tasks of one range
     en->prun([&, k] {
-      rc_tv[k] = plan_intra_A(en, pic, k, n_diag, wctb, hctb);
+      rc_tv[k] = plan_intra_A(en, pic, k);
       if (rc_tv[k]) err_tv[k] = g_err;  // the worker's thread-local message
     });
   for (int part = 0; part < PLAN_PU_PARTS; part++) {
@@ -1466,7 +1356,7 @@ static int plan_and_pack(b200_engine* en, const b200_picture* pic, PicLayout* L,
     if (rc_tv[part]) return set_err(rc_tv[part], "%s", err_tv[part].c_str());
   for (int part = 0; part < PLAN_PU_PARTS; part++)
     if (rc_pu[part]) return set_err(rc_pu[part], "%s", err_pu[part].c_str());
-  plan_intra_finish(en, pic, L, n_diag);
+  plan_intra_finish(en, pic, L);
   merge_list_a(en, L);
   rc = plan_pus_merge(en, pic, L);
   if (rc) return rc;
@@ -1482,8 +1372,6 @@ extern "C" int b200_plan_picture_host(const b200_picture* pic, uint32_t counts[8
   if (!pic || !counts) return set_err(B200_ERR_INVALID, "null argument");
   b200_engine* en = new (std::nothrow) b200_engine();  // no CUDA call is made on this path
   if (!en) return set_err(B200_ERR_NOMEM, "out of memory");
-  if (const char* e = getenv("B200_REGION")) en->region = (atoi(e) == 8) ? 8 : 16;
-  if (const char* e = getenv("B200_INTRA_ORDER")) en->intra_level_order = !strcmp(e, "diag") ? 0 : !strcmp(e, "level_i") ? 1 : 2;
   PicLayout L;
   size_t cap = 0;
   auto now = [] { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
@@ -1497,11 +1385,9 @@ extern "C" int b200_plan_picture_host(const b200_picture* pic, uint32_t counts[8
   t[2] = now();
   t[3] = now();
   if (!rc) {
-    const b200_pic_params& pp = pic->params;
-    const int S = 1 << pp.log2_ctb_size, wctb = (pp.width + S - 1) / S, hctb = (pp.height + S - 1) / S, n_diag = wctb + 2 * hctb;
     plan_intra_ranges(en, pic);
-    for (int k = 0; k < PLAN_INTRA_PARTS && !rc; k++) rc = plan_intra_A(en, pic, k, n_diag, wctb, hctb);
-    if (!rc) plan_intra_finish(en, pic, &L, n_diag);
+    for (int k = 0; k < PLAN_INTRA_PARTS && !rc; k++) rc = plan_intra_A(en, pic, k);
+    if (!rc) plan_intra_finish(en, pic, &L);
   }
   t[4] = now();
   if (prof) {
@@ -1510,11 +1396,7 @@ extern "C" int b200_plan_picture_host(const b200_picture* pic, uint32_t counts[8
     for (int part = 0; part < PLAN_PU_PARTS && !rc; part++) en->pu_ref_mask[part] = 0;
     if (!rc) rc = plan_pus_merge(en, pic, &L);
     u[1] = now();
-    if (!rc) {
-      const b200_pic_params& pp = pic->params;
-      const int S = 1 << pp.log2_ctb_size, wctb = (pp.width + S - 1) / S, hctb = (pp.height + S - 1) / S;
-      plan_intra_finish(en, pic, &L, wctb + 2 * hctb);
-    }
+    if (!rc) plan_intra_finish(en, pic, &L);
     u[2] = now();
     merge_list_a(en, &L);
     u[3] = now();
@@ -1566,7 +1448,7 @@ static bool same_geometry(const Surface& s, const b200_pic_params& p)
 static int phys_for_write(b200_engine* en, int d, int k, const b200_pic_params& p)
 {
   const int cur = en->lmap[d];
-  if (cur >= 0 && (!en->rename || en->n_ctx <= 1 || en->timing || phys_idle(en, cur, k))) return cur;
+  if (cur >= 0 && (en->n_ctx <= 1 || en->timing || phys_idle(en, cur, k))) return cur;
   int best = -1, empty = -1, other = -1;
   for (int ph = 0; ph < B200_MAX_PHYS && best < 0; ph++) {
     if (en->owner[ph] >= 0) continue;
@@ -1749,9 +1631,6 @@ static int pick_ctx(b200_engine* en, uint32_t ref_mask, int dst_slot)
     k = base + en->next_ind % pool;
     en->next_ind = (en->next_ind + 1) % pool;
     depth = en->key_depth + 1;  // what references it comes after the pictures already queued
-  } else if (en->sched_rr) {
-    k = en->next_ctx;
-    en->next_ctx = (en->next_ctx + 1) % en->n_ctx;
   } else {
     int best = -1, shallow = 0;
     for (int c = 0; c < en->n_ctx; c++) {
@@ -1927,12 +1806,8 @@ static int async_start(b200_engine* en)
   try {  // thread creation may throw (resource limits): no exception leaves the C ABI
     as->sequencer = std::thread(async_sequencer, en);
     for (int i = 0; i < n; i++) {
-      b200_engine* sh = new b200_engine();  // no CUDA state: only the planner's scratch and the flags the planner reads
+      b200_engine* sh = new b200_engine();  // no CUDA state: only the planner's scratch
       sh->device = en->device;
-      sh->region = en->region;
-      sh->mc_legacy = en->mc_legacy;
-      sh->intra_split_planes = en->intra_split_planes;
-      sh->intra_level_order = en->intra_level_order;
       sh->helper = &en->pool;
       as->shadows.push_back(sh);
       as->planners.emplace_back(async_planner, en, sh);

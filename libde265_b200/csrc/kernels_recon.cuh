@@ -7,9 +7,9 @@
 //   k_intra<P>      every intra TU: border gather + substitution + smoothing, DC/planar/angular prediction,
 //                   then the TU's residual.  Intra TUs are serially dependent through their neighbours
 //                   (SURVEY §3.2), so the kernel executes the dependency DAG directly: warps claim *tasks*
-//                   through an atomic ticket in a topological order (CTB anti-diagonal x + 2y, then decode
-//                   order).  A task = the TUs (<= 8x8) of one plane inside one aligned 16x16-luma / 8x8-chroma
-//                   region, run in decode order on a shared-memory tile, or one larger TU.  Everything that
+//                   through an atomic ticket in a topological order (DAG level, then decode order; engine.cu
+//                   plan_intra_levels).  A task = the TUs (<= 8x8) of one plane inside one aligned 16x16-luma /
+//                   8x8-chroma region, run in decode order on a shared-memory tile, or one larger TU.  Everything that
 //                   does not depend on the neighbours (TU records, coefficient lists, dequant + inverse
 //                   transform into an int32 residual buffer) is done BEFORE the warp polls the pending flags
 //                   of the neighbour units its availability masks let it read; the dependent part is only
@@ -26,6 +26,8 @@
 #define RC_WARPS 8
 #define RC_THREADS (RC_WARPS * 32)
 #define RC_GSTRIDE 34      // int16 row stride of the first-stage buffer
+#define RC_LG_REGION 4     // intra region task: 16x16 luma / 8x8 chroma samples (the planner's tasks and k_intra's tile)
+#define RC_REGION (1 << RC_LG_REGION)
 #define RC_TILE_STRIDE 40  // region tile: rows -1..2G-1 (only column -1 below row G-1), columns -1..2G-1 (G <= 16)
 #define RC_BLK (33 * RC_TILE_STRIDE + 8)
 #define RC_FULL 0xffffffffu
@@ -35,10 +37,9 @@ struct ReconArgs {
   const uint32_t* list;       // TU indices this launch works on (k_residual: any order; k_intra: grouped by task)
   int n_list;
   int poll_ns;                // k_intra: cap of the polling back-off
-  int region;                 // k_intra: luma size of a region task (16 or 8)
+  int n_task;                 // k_intra: number of tasks
   int n_listw, n_list8;       // k_residual: list = [n_listw warp-per-TU entries | n_list8 8x8 TUs | the rest: 4x4 TUs]
   const uint32_t* task_start; // k_intra: [n_task + 1] offsets into list, tasks in topological order
-  int n_task;
   const b200_coeff* coeffs;
   const uint8_t* scaling;     // B200_SCALING_FACTOR_BYTES or null
   unsigned int* ticket;       // zeroed before launch (k_intra)
@@ -694,15 +695,10 @@ __global__ void __launch_bounds__(RC_THREADS, 3) k_intra(DevPic pic, ReconArgs a
     if (lane < (int)count) tus[lane] = args.tus[args.list[first + lane]];
     __syncwarp();
     const b200_tu tu0 = tus[0];
-    // A task is one large TU, or the small TUs of one region: of one plane, or (pictures with inter prediction) of all planes,
-    // sorted luma | Cb | Cr: up to three SEGMENTS, each with its own plane, tile and dependency frame.
-    const int G0 = args.region >> (tu0.cidx ? 1 : 0);
-    const bool region = (1 << tu0.log2_size) <= min(G0, 8);  // small TUs on a shared-memory tile; larger ones straight from the picture
-    unsigned seg_starts;  // bit i: TU i starts a segment
-    {
-      const int mc = (lane < (int)count) ? tus[lane].cidx : -1, pc = (lane > 0 && lane < (int)count) ? tus[lane - 1].cidx : -1;
-      seg_starts = __ballot_sync(RC_FULL, lane < (int)count && (lane == 0 || mc != pc));
-    }
+    // A task is one large TU, or the small TUs of one plane inside one region
+    const int c = tu0.cidx, G = RC_REGION >> (c ? 1 : 0);
+    const bool region = (1 << tu0.log2_size) <= min(G, 8);  // small TUs on a shared-memory tile; larger ones straight from the picture
+    const int rx = region ? tu0.x & ~(G - 1) : tu0.x, ry = region ? tu0.y & ~(G - 1) : tu0.y;  // dependency frame origin
     {
       // residuals of all the task's TUs, in parallel where the sizes allow: lane i owns TU i's record; 4x4 TUs run one
       // per lane, 8x8 TUs one per quarter-warp, larger ones one after the other on the whole warp.  res holds the TUs'
@@ -742,16 +738,12 @@ __global__ void __launch_bounds__(RC_THREADS, 3) k_intra(DevPic pic, ReconArgs a
                              sm.tb, lane);
       }
     }
-    // ---- wait: one flag per distinct external neighbour unit, one lane each; segment after segment ----
-    for (unsigned ss = seg_starts; ss; ss &= ss - 1) {
-      const int s0 = __ffs(ss) - 1, s1 = (ss & (ss - 1)) ? __ffs(ss & (ss - 1)) - 1 : (int)count;
-      const b200_tu& ts0 = tus[s0];
-      const int c = ts0.cidx, G = args.region >> (c ? 1 : 0);
-      const int rx = region ? ts0.x & ~(G - 1) : ts0.x, ry = region ? ts0.y & ~(G - 1) : ts0.y;  // dependency frame origin
-      const int span = region ? (2 * G) >> 2 : (1 << ts0.log2_size) >> 1;
+    // ---- wait: one flag per distinct external neighbour unit, one lane each ----
+    {
+      const int span = region ? (2 * G) >> 2 : (1 << tu0.log2_size) >> 1;
       unsigned left = 0, top = 0;
       bool corner = false;
-      if (lane >= s0 && lane < s1) dep_units_of(tus[lane], rx, ry, span, left, corner, top);
+      if (lane < (int)count) dep_units_of(tus[lane], rx, ry, span, left, corner, top);
       left = __reduce_or_sync(RC_FULL, left);
       top = __reduce_or_sync(RC_FULL, top);
       corner = __any_sync(RC_FULL, corner);
@@ -794,10 +786,10 @@ __global__ void __launch_bounds__(RC_THREADS, 3) k_intra(DevPic pic, ReconArgs a
     __threadfence();  // acquire: the neighbours' samples were published before their flags were cleared
     if (args.trace) tr_c1 = clock64();
 
+    const int bd = c ? pic.bd_c : pic.bd_y;
+    const bool filter_plane = !(pic.flags & B200_PIC_INTRA_SMOOTHING_OFF) && (c == 0 || pic.chroma == 3);
     if (!region) {
       // ---- one large TU: borders straight from the picture ----
-      const int c = tu0.cidx, bd = c ? pic.bd_c : pic.bd_y;
-      const bool filter_plane = !(pic.flags & B200_PIC_INTRA_SMOOTHING_OFF) && (c == 0 || pic.chroma == 3);
       const int nT = 1 << tu0.log2_size;
       const int gstride = pic.pitch[c] / (int)sizeof(P);
       const P* gsrc = row_ptr<P>(pic.cur[c], pic.pitch[c], tu0.y) + tu0.x;
@@ -809,64 +801,56 @@ __global__ void __launch_bounds__(RC_THREADS, 3) k_intra(DevPic pic, ReconArgs a
       block_store<P>(blk, pic.cur[c], pic.pitch[c], tu0.x, tu0.y, nT, lane);
     } else {
       // ---- regions of small TUs: stage region + top row (2G) + left column (2G) in shared memory, run the TUs in order ----
-      int rbase = 0;
-      for (unsigned ss = seg_starts; ss; ss &= ss - 1) {
-        const int s0 = __ffs(ss) - 1, s1 = (ss & (ss - 1)) ? __ffs(ss & (ss - 1)) - 1 : (int)count;
-        const b200_tu& ts0 = tus[s0];
-        const int c = ts0.cidx, bd = c ? pic.bd_c : pic.bd_y, G = args.region >> (c ? 1 : 0);
-        const int rx = ts0.x & ~(G - 1), ry = ts0.y & ~(G - 1);
-        const bool filter_plane = !(pic.flags & B200_PIC_INTRA_SMOOTHING_OFF) && (c == 0 || pic.chroma == 3);
-        const int pwid = c ? pic.cw : pic.w, phei = c ? pic.ch : pic.h;
-        int covered = 0;  // samples this segment writes
-        for (int i = s0; i < s1; i++) covered += 1 << (2 * tus[i].log2_size);
-        const int TS = RC_TILE_STRIDE;
-        P* tile = blk + TS + 4;  // tile(0,0) = region origin, 4-byte aligned; tile(-1,-1) is blk[3]
-        const int gw = min(G, pwid - rx), gh = min(G, phei - ry);
-        const bool full = (gw == G) && (gh == G);
-        // the interior is only needed where this task does not write it itself (regions partly covered by inter blocks)
-        if (covered < gw * gh) {
-          if (full) {  // whole rows as 4-byte words, like the store below
-            const int wpr = G * (int)sizeof(P) / 4;
-            for (int o = lane; o < G * wpr; o += 32) {
-              const int y = o / wpr, u = o % wpr;  // wpr is a power of two
-              reinterpret_cast<uint32_t*>(tile + y * TS)[u] = __ldcg(reinterpret_cast<const uint32_t*>(row_ptr<P>(pic.cur[c], pic.pitch[c], ry + y) + rx) + u);
-            }
-          } else {
-            for (int o = lane; o < gw * gh; o += 32) {
-              const int x = o % gw, y = o / gw;
-              tile[y * TS + x] = __ldcg(row_ptr<P>(pic.cur[c], pic.pitch[c], ry + y) + rx + x);
-            }
-          }
-        }
-        if (ry > 0)
-          for (int x = lane - 1; x < 2 * G; x += 32)
-            if (rx + x >= 0 && rx + x < pwid) tile[-TS + x] = __ldcg(row_ptr<P>(pic.cur[c], pic.pitch[c], ry - 1) + rx + x);
-        if (rx > 0)  // left column incl. the bottom-left reach (available when the region is a top-left child of its parent block)
-          for (int y = lane; y < 2 * G; y += 32)
-            if (ry + y < phei) tile[y * TS - 1] = __ldcg(row_ptr<P>(pic.cur[c], pic.pitch[c], ry + y) + rx - 1);
-        __syncwarp();
-        for (int i = s0; i < s1; i++) {
-          const b200_tu& tu = tus[i];
-          P* tdst = tile + (tu.y - ry) * TS + (tu.x - rx);
-          const res_t* tres = (tu.flags & B200_TU_CBF) ? res + rbase : nullptr;
-          if (!intra_fast_ok(tu)) tu_intra_small<P>(tu, tdst, TS, bd, filter_plane, tres, lane);
-          else if (tu.log2_size == 2) tu_intra_fast<P, 2>(tu, tdst, TS, bd, filter_plane, tres, lane);
-          else tu_intra_fast<P, 3>(tu, tdst, TS, bd, filter_plane, tres, lane);
-          rbase += 1 << (2 * tu.log2_size);
-        }
-        if (full) {  // whole rows as 4-byte words (tile rows are 4-byte aligned: TS * sizeof(P) and the origin offset are multiples of 4)
-          const int wpr = G * (int)sizeof(P) / 4;  // words per row
+      const int pwid = c ? pic.cw : pic.w, phei = c ? pic.ch : pic.h;
+      int covered = 0;  // samples this task writes
+      for (int i = 0; i < (int)count; i++) covered += 1 << (2 * tus[i].log2_size);
+      const int TS = RC_TILE_STRIDE;
+      P* tile = blk + TS + 4;  // tile(0,0) = region origin, 4-byte aligned; tile(-1,-1) is blk[3]
+      const int gw = min(G, pwid - rx), gh = min(G, phei - ry);
+      const bool full = (gw == G) && (gh == G);
+      // the interior is only needed where this task does not write it itself (regions partly covered by inter blocks)
+      if (covered < gw * gh) {
+        if (full) {  // whole rows as 4-byte words, like the store below
+          const int wpr = G * (int)sizeof(P) / 4;
           for (int o = lane; o < G * wpr; o += 32) {
             const int y = o / wpr, u = o % wpr;  // wpr is a power of two
-            reinterpret_cast<uint32_t*>(row_ptr<P>(pic.cur[c], pic.pitch[c], ry + y) + rx)[u] = reinterpret_cast<const uint32_t*>(tile + y * TS)[u];
+            reinterpret_cast<uint32_t*>(tile + y * TS)[u] = __ldcg(reinterpret_cast<const uint32_t*>(row_ptr<P>(pic.cur[c], pic.pitch[c], ry + y) + rx) + u);
           }
         } else {
           for (int o = lane; o < gw * gh; o += 32) {
             const int x = o % gw, y = o / gw;
-            row_ptr<P>(pic.cur[c], pic.pitch[c], ry + y)[rx + x] = tile[y * TS + x];
+            tile[y * TS + x] = __ldcg(row_ptr<P>(pic.cur[c], pic.pitch[c], ry + y) + rx + x);
           }
         }
-        __syncwarp();  // the tile is reused by the next segment
+      }
+      if (ry > 0)
+        for (int x = lane - 1; x < 2 * G; x += 32)
+          if (rx + x >= 0 && rx + x < pwid) tile[-TS + x] = __ldcg(row_ptr<P>(pic.cur[c], pic.pitch[c], ry - 1) + rx + x);
+      if (rx > 0)  // left column incl. the bottom-left reach (available when the region is a top-left child of its parent block)
+        for (int y = lane; y < 2 * G; y += 32)
+          if (ry + y < phei) tile[y * TS - 1] = __ldcg(row_ptr<P>(pic.cur[c], pic.pitch[c], ry + y) + rx - 1);
+      __syncwarp();
+      int rbase = 0;
+      for (int i = 0; i < (int)count; i++) {
+        const b200_tu& tu = tus[i];
+        P* tdst = tile + (tu.y - ry) * TS + (tu.x - rx);
+        const res_t* tres = (tu.flags & B200_TU_CBF) ? res + rbase : nullptr;
+        if (!intra_fast_ok(tu)) tu_intra_small<P>(tu, tdst, TS, bd, filter_plane, tres, lane);
+        else if (tu.log2_size == 2) tu_intra_fast<P, 2>(tu, tdst, TS, bd, filter_plane, tres, lane);
+        else tu_intra_fast<P, 3>(tu, tdst, TS, bd, filter_plane, tres, lane);
+        rbase += 1 << (2 * tu.log2_size);
+      }
+      if (full) {  // whole rows as 4-byte words (tile rows are 4-byte aligned: TS * sizeof(P) and the origin offset are multiples of 4)
+        const int wpr = G * (int)sizeof(P) / 4;  // words per row
+        for (int o = lane; o < G * wpr; o += 32) {
+          const int y = o / wpr, u = o % wpr;  // wpr is a power of two
+          reinterpret_cast<uint32_t*>(row_ptr<P>(pic.cur[c], pic.pitch[c], ry + y) + rx)[u] = reinterpret_cast<const uint32_t*>(tile + y * TS)[u];
+        }
+      } else {
+        for (int o = lane; o < gw * gh; o += 32) {
+          const int x = o % gw, y = o / gw;
+          row_ptr<P>(pic.cur[c], pic.pitch[c], ry + y)[rx + x] = tile[y * TS + x];
+        }
       }
     }
     __threadfence();  // release: samples before flags

@@ -13,7 +13,7 @@ from libde265_b200 import capi, synth
 AVAIL_CORNER, AVAIL_TOP0 = 16, 17
 
 
-def plan(lib, pic, region=16):
+def plan(lib, pic):
     cp = pic.c
     counts = (C.c_uint32 * 8)()
     n_tu, n_pu = len(pic.tus), len(pic.pus)
@@ -73,29 +73,21 @@ def check_picture(lib, pic):
     assert ts[0] == 0 and ts[-1] == len(lb) and (np.diff(ts.astype(np.int64)) >= 1).all() and (np.diff(ts.astype(np.int64)) <= 16).all()
     owner = [np.full(((pic.params.height >> (1 if c else 0)) // 4 + 1, (pic.params.width >> (1 if c else 0)) // 4 + 1), -1, np.int64) for c in range(3)]
     task_of = {}
-    merged = len(pus) > 0  # pictures with inter prediction: the small TUs of ALL planes of a region form one task (luma | Cb | Cr)
-    n_merged = 0
     for t in range(len(ts) - 1):
         members = lb[ts[t]:ts[t + 1]]
-        planes = [int(tus["cidx"][i]) for i in members]
-        assert planes == sorted(planes), "planes in the order luma, Cb, Cr inside a task"
-        if len(set(planes)) > 1:
-            assert merged
-            n_merged += 1
-        rx0, ry0 = (int(tus["x"][members[0]]) << (1 if planes[0] else 0)) // 16, (int(tus["y"][members[0]]) << (1 if planes[0] else 0)) // 16
-        for c0 in sorted(set(planes)):
-            seg = np.array([i for i in members if int(tus["cidx"][i]) == c0])
-            G = 16 >> (1 if c0 else 0)
-            assert (np.diff(seg.astype(np.int64)) > 0).all(), "decode order inside a plane of a task"
-            for i in seg:
-                tu = tus[i]
-                nT = 1 << int(tu["log2_size"])
-                if len(members) > 1:
-                    sh = 1 if c0 else 0
-                    assert nT < G and (int(tu["x"]) << sh) // 16 == rx0 and (int(tu["y"]) << sh) // 16 == ry0
-                task_of[int(i)] = t
-                owner[c0][int(tu["y"]) // 4:(int(tu["y"]) + nT) // 4, int(tu["x"]) // 4:(int(tu["x"]) + nT) // 4] = t
-    assert merged or n_merged == 0
+        planes = {int(tus["cidx"][i]) for i in members}
+        assert len(planes) == 1, f"task {t} mixes planes {sorted(planes)}"
+        c0 = planes.pop()
+        sh, G = (1 if c0 else 0), 16 >> (1 if c0 else 0)
+        rx0, ry0 = (int(tus["x"][members[0]]) << sh) // 16, (int(tus["y"][members[0]]) << sh) // 16
+        assert (np.diff(members.astype(np.int64)) > 0).all(), "decode order inside a task"
+        for i in members:
+            tu = tus[i]
+            nT = 1 << int(tu["log2_size"])
+            if len(members) > 1:
+                assert nT < G and (int(tu["x"]) << sh) // 16 == rx0 and (int(tu["y"]) << sh) // 16 == ry0
+            task_of[int(i)] = t
+            owner[c0][int(tu["y"]) // 4:(int(tu["y"]) + nT) // 4, int(tu["x"]) // 4:(int(tu["x"]) + nT) // 4] = t
     # ---- topological order ----
     for i, t in task_of.items():
         tu = tus[i]

@@ -147,21 +147,6 @@ def test_synthetic_sequence_every_stage(eng, oracle_mod, bd):
     orc.close()
 
 
-def test_intra_task_and_ticket_variants(oracle_mod, monkeypatch):
-    """The non-default shapes of the intra work list stay exact: planes of a region merged into one task (B200_INTRA_SPLIT=0) and
-    CTB anti-diagonal ticket order (B200_INTRA_ORDER=diag)."""
-    for env in ({"B200_INTRA_SPLIT": "0"}, {"B200_INTRA_ORDER": "diag"}, {"B200_INTRA_SPLIT": "0", "B200_INTRA_ORDER": "diag"}):
-        for k, v in env.items():
-            monkeypatch.setenv(k, v)
-        e = Engine(0)
-        orc = oracle_mod.Oracle()
-        run_sequence(e, orc, 416, 240, 8)
-        orc.close()
-        e.close()
-        for k in env:
-            monkeypatch.delenv(k)
-
-
 @pytest.mark.parametrize("size", [(8, 8), (16, 8), (72, 40), (64, 64), (200, 136), (1288, 8)])
 def test_ragged_and_tiny_pictures(eng, oracle_mod, size):
     """Pictures that are not a multiple of the CTB size, down to a single minimum CB."""
